@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- mpileup reference positions/sec on the BASELINE workloads.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--region-mb M] [--modes a,b,...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--region-mb M] [--modes a,b,...] [--dump-outputs DIR]
   (N>1: python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...)
 
 ONE JSON line.  Its top-level keys are the headline workload; `modes` holds one sub-record per further
@@ -18,6 +18,8 @@ A "step" is one pass of the hot path over one staged batch; inputs (0.05 GB/Mb) 
 step are far larger than the 126 MB L2, so successive steps cannot be served from cache.  With N GPUs every
 rank owns its own region (weak scaling, no data-path collective; the one collective is the all_gather of the
 per-region column summaries rank 0 needs to emit shards in genome order, issued once for all timed steps).
+Every workload runs K timed steps.  Inputs are generated from fixed seeds, so the same arguments give the same
+inputs on every run, and --dump-outputs lets two builds be compared output for output.
 
 value  device-resident: inputs already staged in HBM; K x (read stage + column stage), max over ranks.
 e2e    through the C ABI with HOST buffers: pinned-host SoA -> b200_stage (H2D + read stage) ->
@@ -238,6 +240,37 @@ def panel_columns(p):
     return int((seg_end - seg_beg).sum())
 
 
+def text_arrays(name, text, seed, runs=32, run_len=1 << 16, block=1 << 20):
+    """A text output as arrays small enough to store: its length; two checksums per MiB over all of it (the byte sum and the
+    sum weighted by the position in the MiB, both exact in float64); `runs` stretches of `run_len` bytes at seeded offsets,
+    byte values as float32."""
+    a = np.frombuffer(text, np.uint8)
+    w = 1 + np.arange(block, dtype=np.int64) % 65521
+    sums = np.zeros((-(-len(a) // block), 2), np.float64)
+    for i in range(len(sums)):
+        seg = a[i * block:(i + 1) * block].astype(np.int64)
+        sums[i] = seg.sum(), seg @ w[:len(seg)]
+    starts = np.sort(np.random.default_rng(seed).integers(0, max(1, len(a) - run_len + 1), runs))
+    sample = np.concatenate([a[s:s + run_len] for s in starts]).astype(np.float32)
+    return {f'{name}_length': np.array([len(a)], np.float64), f'{name}_checksums': sums, f'{name}_sample': sample}
+
+
+def gl_arrays(name, pos, n, qs, p25, seed, rows=1 << 15):
+    """Genotype-likelihood columns as arrays: per-field sums over every column (float64) and a seeded sample of columns."""
+    k = len(pos)
+    idx = np.sort(np.random.default_rng(seed).choice(k, min(k, rows), replace=False))
+    sums = np.concatenate([[k, n.sum()], qs.reshape(k, -1).sum(0, dtype=np.float64), p25.reshape(k, -1).sum(0, dtype=np.float64)])
+    return {f'{name}_sums': sums.astype(np.float64), f'{name}_pos': pos[idx].astype(np.float64), f'{name}_n': n[idx].astype(np.float64),
+            f'{name}_qsum': qs[idx].astype(np.float32), f'{name}_p25': p25[idx].astype(np.float32)}
+
+
+def write_dump(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(d, name + '.npy'), a)
+
+
 def run_oracle_parallel(exe, argv, procs):
     t0 = time.perf_counter()
     ps = [subprocess.Popen([exe] + argv, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL) for _ in range(procs)]
@@ -332,6 +365,9 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--e2e-handles', type=int, default=4,
                     help='engine handles (one host thread each) used by the end-to-end loop; handles are per-thread objects like the htslib iterators they replace')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last step of each workload returned to its caller as DIR/<name>.npy '
+                         '(float32/float64; text outputs as length, per-MiB checksums and a seeded sample; rank 0 only)')
     args = ap.parse_args()
     if args.impl == 'reference':
         return reference_arm(args)
@@ -415,7 +451,7 @@ def main():
         return n.value
 
     def run_e2e(k_steps):
-        """k_steps windows through n_h handles; returns bytes of the last window"""
+        """k_steps windows through n_h handles; returns the text bytes of each handle's last window"""
         res = [0] * n_h
         def worker(j):
             for s_ in range(j, k_steps, n_h):
@@ -424,7 +460,7 @@ def main():
         ths = [_th.Thread(target=worker, args=(j,)) for j in range(n_h)]
         [t.start() for t in ths]; [t.join() for t in ths]
         exchange_summaries()
-        return max(res)
+        return res
 
     for _ in range(args.warmup):
         run_e2e(n_h); step_device()
@@ -448,9 +484,13 @@ def main():
         # ---- end to end through the C ABI with host buffers
         sync_all()
         t0 = time.perf_counter()
-        run_e2e(args.steps)
+        e2e_bytes = run_e2e(args.steps)
         sync_all()
         dt_e2e = time.perf_counter() - t0
+    dump = {}
+    if args.dump_outputs and rank == 0:
+        last = (args.steps - 1) % n_h                 # the handle that ran the last timed window
+        dump.update(text_arrays('mpileup_a_text', outs[last][:e2e_bytes[last]], seed=1))
     dt = shard.max_over_ranks(dt, dev); dt_e2e = shard.max_over_ranks(dt_e2e, dev)
     clocks = clk.summary()
     for h in handles[1:]:
@@ -489,7 +529,7 @@ def main():
 
     # ------------------------------------------------------------------------------------ further BASELINE configurations
     sub = {}
-    msteps = max(3, min(args.steps, 10))
+    msteps = args.steps
 
     def timed(fn, k, w=2):
         for _ in range(w):
@@ -526,6 +566,8 @@ def main():
                          'peak_source': 'nominal: 148 SMs x 64 FP64 lanes x 1.965 GHz (no measured FP64 figure in MEASURED_PEAKS.json)',
                          'algorithmic_ops_per_launch': ops, 'kernel_ms': bms, 'traffic': None,
                          'step_kernels_ms': {'read_stage_total': float(np.mean(st_ms[-msteps:])), 'of_which_baq': bms, 'column_stage': float(np.mean(k_ms[-msteps:]))}}}
+        if args.dump_outputs and rank == 0:           # the column stage again on the last step's staged reads: same bytes
+            dump.update(text_arrays('mpileup_f_baq_text', e.mpileup_text(mconf), seed=2))
         e.close()
 
     if 'depth_a' in modes or 'coverage' in modes:
@@ -548,15 +590,21 @@ def main():
                                            'unit': 'GB/s', 'frac': (din + dlen) / (kd * 1e-3) / 1e9 / peak, 'peak_source': peak_src,
                                            'algorithmic_bytes_per_launch': int(din + dlen), 'kernel_ms': kd, 'traffic': None,
                                            'step_kernels_ms': {'read_stage': float(np.mean(st_ms[-msteps:])), 'column_stage': kd}}}
+            if args.dump_outputs and rank == 0:
+                dump.update(text_arrays('depth_a_text', e.depth_text(all=1), seed=3))
         if 'coverage' in modes:
             cconf = engine.default_stage_conf(engine.MODE_COVERAGE, rflag_filter=4 | 256 | 512 | 1024, end=ncols)
             e.stage(soa, cconf)
             k_ms, st_ms = [], []
+            cov = {}
 
             def step_cov():
-                e.restage(); st_ms.append(e.last_stage_device_ms)
-                e.coverage(min_baseQ=0, min_depth=1); k_ms.append(e.last_kernel_ms)
+                st = e.restage(); st_ms.append(e.last_stage_device_ms)
+                cov.update(e.coverage(min_baseQ=0, min_depth=1), n_selected_reads=st.n_selected_reads, summed_mapq=st.summed_mapq)
+                k_ms.append(e.last_kernel_ms)
             dtc = timed(step_cov, msteps)
+            if args.dump_outputs and rank == 0:
+                dump['coverage_sums'] = np.array(list(cov.values()), np.float64)
             cin = int((soa['l_qseq'].astype(np.int64) + 4 * soa['n_cigar'].astype(np.int64) + 24).sum())   # qualities + cigar + core fields
             kc = float(np.mean(k_ms[-msteps:]))
             sub['coverage'] = {'workload': f'`coverage` over the same {args.region_mb:g} Mb window (BASELINE config 5)',
@@ -589,6 +637,16 @@ def main():
                                      'frac': (gin + gout) / (kg * 1e-3) / 1e9 / peak, 'peak_source': peak_src, 'algorithmic_bytes_per_launch': int(gin + gout),
                                      'kernel_ms': kg, 'traffic': None, 'step_kernels_ms': {'read_stage': float(np.mean(st_ms[-msteps:])), 'column_stage': kg}}}
         e.close()
+        if args.dump_outputs and rank == 0:
+            # errmod_cal's shuffle draws from one random stream that runs on across calls, so a fresh handle makes as many calls
+            # as preceded the last timed step (one warm-up, msteps - 1 timed) before it fetches that step's columns
+            r = engine.Engine(local); r.set_keep_raw(True)
+            st = r.stage(pp, gconf)
+            for _ in range(msteps):
+                r.restage(); r.glf(13, 0, fetch=False)
+            r.restage()
+            dump.update(gl_arrays('gl_c4', *r.glf(13, int(st.n_cols) + 16), seed=4))
+            r.close()
 
     if rank == 0:
         if world == 1 and not args.no_cpu_baseline:
@@ -601,6 +659,8 @@ def main():
                     rec, _ = cpu_leg(exe, sample, m, 1, 1, 0)
                     sub[m]['cpu_baseline'] = rec
         line['modes'] = sub
+        if args.dump_outputs:
+            write_dump(args.dump_outputs, dump)
         print(json.dumps(line))
     eng.close(); eng_dev.close()
     if world > 1:

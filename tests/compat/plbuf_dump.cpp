@@ -1,6 +1,7 @@
-// plbuf_dump.cpp -- client of the reference's own bam_plbuf layer (bam_plbuf.h:32-51), which is compiled UNMODIFIED from
-// /root/reference/bam_plbuf.c against tests/compat/shim/htslib/sam.h -> include/b200_htslib_compat.h.  Shows that the
-// in-tree layer riding on the iterator API keeps working (SURVEY.md section 8b).  Same dump format as plp_dump.
+// plbuf_dump.cpp -- client of samtools' own bam_plbuf layer (bam_plbuf.h:32-51), which is compiled UNMODIFIED from a
+// samtools source tree against tests/compat/shim/htslib/sam.h -> include/b200_htslib_compat.h by
+// tests/golden/make_plbuf_golden.py.  Shows that the layer riding on the iterator API keeps working (SURVEY.md section 8b).
+// Same dump format as plp_dump.
 #include "fill_bam1.hpp"
 #include <cstdio>
 extern "C" {

@@ -17,18 +17,10 @@ g++ -std=c++17 -O1 -g -ffp-contract=off -Wall -Wno-unused-function -o tests/emul
 # the htslib-compatible iterator tier (plp_compat.cpp) + its test client, on the emulation harness
 g++ -std=c++17 -O1 -g -ffp-contract=off -Wall -Wno-unused-function -Iinclude -o tests/emul/_build/plp_dump_emul.tmp$$ \
     tests/compat/plp_dump.cpp samtools_b200/csrc/host/plp_compat.cpp samtools_b200/csrc/host/hts_io.cpp tests/emul/emul_engine.cpp -lz
-# the reference's own bam_plbuf layer, compiled UNMODIFIED where it lies (only in the dev container: /root/reference does
-# not travel) against tests/compat/shim/htslib/sam.h -> include/b200_htslib_compat.h; outputs stay under _build/
-REF=${B200_REFERENCE_DIR:-/root/reference}
-if [ -f "$REF/bam_plbuf.c" ]; then
-    gcc -c -O1 -Itests/compat/shim -Iinclude -I"$REF" -o tests/emul/_build/ref_bam_plbuf.o.tmp$$ "$REF/bam_plbuf.c"
-    g++ -std=c++17 -O1 -g -Iinclude -Itests/compat/shim -I"$REF" -o tests/emul/_build/plbuf_dump_emul.tmp$$ tests/compat/plbuf_dump.cpp \
-        tests/emul/_build/ref_bam_plbuf.o.tmp$$ samtools_b200/csrc/host/plp_compat.cpp samtools_b200/csrc/host/hts_io.cpp tests/emul/emul_engine.cpp -lz
-fi
 # the register-band BAQ arithmetic (samtools_b200/csrc/baq_reg.h) single-stepped on the CPU against the oracle's sam_prob_realn
 make -s -C oracle
 g++ -std=c++17 -O2 -ffp-contract=off -Wno-unknown-pragmas -o tests/emul/_build/baq_host.tmp$$ tests/emul/baq_host.cpp \
     -Loracle/_build -loracle -Wl,-rpath,"$PWD/oracle/_build" -lz -lm
 
-for f in b200samtools_emul baq_host plbuf_dump_emul plp_dump_emul ref_bam_plbuf.o; do if [ -f tests/emul/_build/$f.tmp$$ ]; then mv -f tests/emul/_build/$f.tmp$$ tests/emul/_build/$f; fi; done
+for f in b200samtools_emul baq_host plp_dump_emul; do mv -f tests/emul/_build/$f.tmp$$ tests/emul/_build/$f; done
 mv -f tests/emul/_build/.stamp.new.$$ tests/emul/_build/.stamp

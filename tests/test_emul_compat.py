@@ -1,7 +1,7 @@
 """The htslib-compatible iterator tier (samtools_b200/csrc/host/plp_compat.cpp) on the emulation harness: the host logic of
 bam_plp_* / bam_mplp_* (contig buffering, k-way merge, slab paging, hooks) against the oracle's restatement of htslib's
 iterator, without a GPU.  The same cases run on the CUDA engine in tests/test_gpu_parity.py::test_htslib_compat_iterator."""
-import os, subprocess
+import hashlib, json, os, subprocess
 import pytest
 import golden_cases
 from conftest import ROOT
@@ -35,18 +35,20 @@ def test_iterator_hooks_and_kstring_insertion(args, files, dump_emul, oracle_bin
     assert b'hooks: ctor=' in got.stderr and b'bad=0' in got.stderr
 
 
-@pytest.mark.parametrize('f', ['test/mpileup/mp_DI.sam', 'test/mpileup/mp_N2.sam', 'test/mpileup/mpileup.1.bam'])
+PLBUF_GOLDEN = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'plbuf_dumps.json')))
+
+
+@pytest.mark.parametrize('f', sorted(PLBUF_GOLDEN))
 def test_reference_bam_plbuf_rides_on_the_tier(f, dump_emul, oracle_bin, corpus):
-    """The reference's own bam_plbuf.c (bam_plbuf.h:32-51), compiled unmodified against the compatibility header, drives
-    the iterator tier through bam_plp_push / bam_plp64_next and sees the columns htslib would hand it.  Needs the
-    reference tree, so it runs in the dev container only."""
-    exe = os.path.join(ROOT, 'tests', 'emul', '_build', 'plbuf_dump_emul')
-    if not os.path.exists(exe) or not os.path.exists(os.environ.get('B200_REFERENCE_DIR', '/root/reference') + '/bam_plbuf.c'):
-        pytest.skip('reference tree not present (GPU box): bam_plbuf.c cannot be compiled here')
-    got = subprocess.run([exe, os.path.join(corpus, f)], capture_output=True)
+    """samtools' own bam_plbuf layer (bam_plbuf.h:32-51) drives the iterator tier through bam_plp_push / bam_plp64_next.
+    plp_dump -p drives it the same way (drain after every push, NULL push at the end) and must yield byte for byte the
+    columns bam_plbuf.c saw when it was compiled unmodified against the compatibility header
+    (tests/golden/plbuf_dumps.json, written by tests/golden/make_plbuf_golden.py) and those of htslib's iterator."""
+    got = subprocess.run([dump_emul, '-p', os.path.join(corpus, f)], capture_output=True)
     want = subprocess.run([oracle_bin, 'pileup-dump', os.path.join(corpus, f)], capture_output=True)
     assert got.returncode == 0, got.stderr[-300:]
     assert got.stdout == want.stdout and len(got.stdout) > 100
+    assert {'sha256': hashlib.sha256(got.stdout).hexdigest(), 'bytes': len(got.stdout)} == PLBUF_GOLDEN[f]
 
 
 @pytest.mark.parametrize('budget', ['1', '400', '5000'])
