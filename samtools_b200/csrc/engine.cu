@@ -29,12 +29,12 @@
 #include <string>
 #include <vector>
 #include <algorithm>
-#include <queue>
 
 #include "../../include/b200_pileup.h"
 #include "plp_core.h"
 #include "plp_stage.h"
 #include "engine_internal.h"
+#include "stage_host.h"
 
 using namespace plp;
 
@@ -225,49 +225,29 @@ __global__ void k_scan_max(const int32_t *in, int32_t *out, int64_t n, uint64_t 
     for (int j = 0; j < IPT; ++j) if (base + j < n) out[base + j] = max(pre, v[j]);
 }
 
-// per 32-column group: the [lo,hi) slice of each file's reads that can cover it.
-// lo is the later of (a) the first read whose running max end exceeds the group start and
-// (b) the first read starting within kReach columns of it; reads before (b) that still
-// reach the group are listed separately (k_ovf_*), so one spliced read cannot widen the
-// slice of every group under it.
+// per 32-column group: the [lo,hi) slice of each file's reads that can cover it (group_slice)
 __global__ void k_ranges(const ReadDesc *desc, const int32_t *pmax, const int64_t *file_start, int n_files,
                          int32_t n_groups, int32_t *glo, int32_t *ghi, int *max_range)
 {
     int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (int64_t)n_groups * n_files) return;
     const int f = (int)(idx / n_groups), g = (int)(idx % n_groups);
-    const int64_t fs = file_start[f], fe = file_start[f + 1];
-    const int32_t c0 = g * 32, c1 = c0 + 31;
-    int64_t lo = fs, hi = fe;
-    while (lo < hi) { int64_t m = (lo + hi) >> 1; if (pmax[m] > c0) hi = m; else lo = m + 1; }   // first read whose running max end exceeds c0
-    int64_t first = lo;
-    lo = first; hi = fe;
-    while (lo < hi) { int64_t m = (lo + hi) >> 1; if (desc[m].rpos > c0 - kReach) hi = m; else lo = m + 1; }  // first read within reach
-    if (lo > first) first = lo;
-    lo = first; hi = fe;
-    while (lo < hi) { int64_t m = (lo + hi) >> 1; if (desc[m].rpos > c1) hi = m; else lo = m + 1; }  // first read starting beyond c1
-    const int64_t last = lo > first ? lo : first;
+    int64_t first, last;
+    group_slice(desc, pmax, file_start[f], file_start[f + 1], g, first, last);
     glo[idx] = (int32_t)first;
     ghi[idx] = (int32_t)last;
     atomicMax(max_range, (int)(last - first));
 }
 
-// far-reaching reads: read i is listed for group g when 32g >= rpos_i + kReach and 32g < rend_i
-__device__ __forceinline__ void ovf_span(const ReadDesc &d, int32_t n_groups, int32_t &g0, int32_t &g1)
-{
-    const int64_t a = (int64_t)d.rpos + kReach;
-    g0 = (int32_t)(a <= 0 ? 0 : (a + 31) >> 5);
-    g1 = d.rend > 0 ? (d.rend - 1) >> 5 : -1;
-    if (g1 >= n_groups) g1 = n_groups - 1;
-}
+// far-reaching reads per group (ovf_span)
 __global__ void k_ovf_count(const ReadDesc *desc, const int64_t *file_start, int n_files, int64_t n, int32_t n_groups, uint32_t *cnt)
 {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const ReadDesc d = desc[i];
-    if ((int64_t)d.rend - d.rpos <= kReach) return;
+    int32_t g0, g1;
+    if (!ovf_span(d, n_groups, g0, g1)) return;
     int f = 0; while (f + 1 < n_files && i >= file_start[f + 1]) ++f;
-    int32_t g0, g1; ovf_span(d, n_groups, g0, g1);
     for (int32_t g = g0; g <= g1; ++g) atomicAdd(&cnt[(int64_t)f * n_groups + g], 1u);
 }
 __global__ void k_ovf_fill(const ReadDesc *desc, const int64_t *file_start, int n_files, int64_t n, int32_t n_groups,
@@ -276,9 +256,9 @@ __global__ void k_ovf_fill(const ReadDesc *desc, const int64_t *file_start, int 
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const ReadDesc d = desc[i];
-    if ((int64_t)d.rend - d.rpos <= kReach) return;
+    int32_t g0, g1;
+    if (!ovf_span(d, n_groups, g0, g1)) return;
     int f = 0; while (f + 1 < n_files && i >= file_start[f + 1]) ++f;
-    int32_t g0, g1; ovf_span(d, n_groups, g0, g1);
     for (int32_t g = g0; g <= g1; ++g) {
         const int64_t k = (int64_t)f * n_groups + g;
         idx[off[k] + (int32_t)atomicAdd(&cursor[k], 1u)] = (int32_t)i;
@@ -394,38 +374,7 @@ __global__ void __launch_bounds__(TILE) k_mpileup_write(MpFmt fmt, const uint32_
 #include "mpileup_ss.cuh"
 #include "mpileup_ent.cuh"
 
-// depth rows "name\tpos(\tdepth)*\n" (bam2depth.c:234-244)
-struct DpFmt {
-    View v; DpConf cf;
-    struct State { int32_t d0; };
-    __device__ __forceinline__ uint32_t size(int32_t c, State &s) const
-    {
-        bool any = false; uint32_t body = 0;
-        for (int f = 0; f < v.n_files; ++f) {
-            DpCol o; dp_file_column(v, cf, f, c >> 5, c, o);
-            if (f == 0) s.d0 = o.depth;
-            any |= o.spanned;
-            body += 1 + (uint32_t)ndigits((uint64_t)o.depth);
-        }
-        if (!any && !(cf.all && c < v.ncols_all)) return 0;
-        if (!bed_pass(v, c)) return 0;
-        return (uint32_t)v.name_len + 1 + (uint32_t)ndigits((uint64_t)(v.win_base + c + 1)) + body + 1;
-    }
-    __device__ __forceinline__ void write(int32_t c, const State &s, char *p) const
-    {
-        for (int i = 0; i < v.name_len; ++i) *p++ = v.name[i];
-        *p++ = '\t';
-        p += put_u64(p, (uint64_t)(v.win_base + c + 1));
-        for (int f = 0; f < v.n_files; ++f) {
-            int32_t d = s.d0;
-            if (f) { DpCol o; dp_file_column(v, cf, f, c >> 5, c, o); d = o.depth; }
-            *p++ = '\t';
-            p += put_u64(p, (uint64_t)d);
-        }
-        *p = '\n';
-    }
-};
-
+// depth rows: DpFmt (plp_core.h)
 __global__ void __launch_bounds__(TILE) k_depth_size(DpFmt fmt, uint32_t *len, DpFmt::State *st, uint32_t *tile_total)
 {
     text_size_tile(fmt, fmt.v.ncols, len, st, tile_total);
@@ -469,40 +418,21 @@ __global__ void __launch_bounds__(256) k_coverage_hist(View v, int32_t min_baseQ
     const int32_t c = (int32_t)(blockIdx.x * blockDim.x + threadIdx.x);
     if (c >= v.ncols) return;
     CvCol o; cv_column(v, min_baseQ, c >> 5, c, o);
-    const uint32_t add = plot_depth ? o.depth : ((o.count_base && o.depth >= (uint32_t)min_depth) ? 1u : 0u);
+    const uint32_t add = cv_hist_add(o, min_depth, plot_depth);
     if (!add) return;
     const int64_t bin = ((int64_t)c - beg_rel) / bin_width;
     if (bin >= 0 && bin < n_bins) atomicAdd(&hist[bin], add);
 }
 
 // bedcov column reducers (bedcov.c:316-331) over the staged window, per input file: sum of the per-column depth (optionally
-// without deletions / reference skips) and the number of columns at or above a depth threshold.  A column takes part when
-// the multi-file iterator would return it, i.e. when any file has a read over it.
+// without deletions / reference skips) and the number of columns at or above a depth threshold (bc_any, bc_depth).
 __global__ void __launch_bounds__(256) k_bedcov(View v, int skip_dn, int min_depth, unsigned long long *sums /* [n_files][2] */)
 {
     const int32_t c = (int32_t)(blockIdx.x * blockDim.x + threadIdx.x);
-    const bool live = c < v.ncols;
-    bool any = false;
-    if (live)
-        for (int f = 0; f < v.n_files && !any; ++f) {
-            const ReadRange rr = read_range(v, f, c >> 5);
-            for (int32_t t_ = 0; t_ < rr.n && !any; ++t_) { const ReadDesc d = load_hot(v.desc + range_at(rr, t_)); any = (uint32_t)(c - d.rpos) < (uint32_t)(d.rend - d.rpos); }
-        }
+    const bool any = c < v.ncols && bc_any(v, c);
     for (int f = 0; f < v.n_files; ++f) {
         unsigned long long pd = 0, ge = 0;
-        if (live && any) {
-            const ReadRange rr = read_range(v, f, c >> 5);
-            int32_t np = 0, m = 0;
-            for (int32_t t_ = 0; t_ < rr.n; ++t_) {
-                const int32_t i = range_at(rr, t_);
-                ReadDesc d = load_hot(v.desc + i);
-                if ((uint32_t)(c - d.rpos) >= (uint32_t)(d.rend - d.rpos)) continue;
-                ++np;
-                if (skip_dn && !(d.fl & RD_SIMPLE)) { load_cold(d, v.desc + i); Ent e; resolve(v, d, c, e); if (e.is_del || e.is_refskip) ++m; }
-            }
-            pd = (unsigned long long)(np - m);
-            ge = (min_depth >= 0 && np - m >= min_depth) ? 1ull : 0ull;
-        }
+        if (any) { const int32_t d = bc_depth(v, f, c, skip_dn); pd = (unsigned long long)d; ge = (min_depth >= 0 && d >= min_depth) ? 1ull : 0ull; }
         for (int o = 16; o; o >>= 1) { pd += __shfl_xor_sync(0xffffffffu, pd, o); ge += __shfl_xor_sync(0xffffffffu, ge, o); }
         if ((threadIdx.x & 31) == 0) { if (pd) atomicAdd(&sums[2 * f], pd); if (ge) atomicAdd(&sums[2 * f + 1], ge); }
     }
@@ -513,34 +443,13 @@ __global__ void k_entries_count(View v, int f, int32_t c0, uint32_t *col_n)   //
 {
     const int32_t c = c0 + (int32_t)(blockIdx.x * blockDim.x + threadIdx.x);
     if (c >= v.ncols) return;
-    const int g = c >> 5;
-    const ReadRange rr = read_range(v, f, g);
-    uint32_t n = 0;
-    for (int32_t t_ = 0; t_ < rr.n; ++t_) { const ReadDesc d = v.desc[range_at(rr, t_)]; if (c >= d.rpos && c < d.rend) ++n; }
-    col_n[c - c0] = n;
+    col_n[c - c0] = column_entries<false>(v, f, c, nullptr);
 }
 __global__ void k_entries_fill(View v, int f, int32_t c0, const uint64_t *col_off, b200_pileup1_t *ents)
 {
     const int32_t c = c0 + (int32_t)(blockIdx.x * blockDim.x + threadIdx.x);
     if (c >= v.ncols) return;
-    const int g = c >> 5;
-    const ReadRange rr = read_range(v, f, g);
-    b200_pileup1_t *o = ents + col_off[c - c0];
-    for (int32_t t_ = 0; t_ < rr.n; ++t_) {
-        const int32_t i = range_at(rr, t_);
-        const ReadDesc d = v.desc[i];
-        if (c < d.rpos || c >= d.rend) continue;
-        Ent e; resolve(v, d, c, e);
-        if (e.k < 0) {   // simple read: the op index of its match
-            const uint32_t *cg = v.cigar + d.cig_off; int k = 0;
-            while (!is_mop(cg[k] & 0xf)) ++k;
-            e.k = k;
-        }
-        b200_pileup1_t p;
-        p.read = i; p.qpos = e.qpos; p.indel = e.indel; p.cigar_ind = e.k;
-        p.is_del = e.is_del; p.is_head = e.is_head; p.is_tail = e.is_tail; p.is_refskip = e.is_refskip;
-        *o++ = p;
-    }
+    column_entries<true>(v, f, c, ents + col_off[c - c0]);
 }
 __global__ void k_scan_u32_to_u64(const uint32_t *in, uint64_t *out, int32_t n, uint64_t *st, uint32_t *ticket)
 {
@@ -708,32 +617,24 @@ static int max_buffered_reads(b200_engine *e, int *out)
     return 0;
 }
 
-// max-depth rule of bam_plp_push, evaluated on the host only when a column could
-// hold more than maxcnt reads (sequential by nature; see DESIGN.md).
-static int apply_maxcnt_host(b200_engine *e, int64_t n, int maxcnt)
+// descriptors and states of the staged reads, copied to the host for the host-side rules (stage_host.h)
+static int fetch_desc_state(b200_engine *e, int64_t n, std::vector<ReadDesc> &hd, std::vector<uint8_t> &st)
 {
-    std::vector<ReadDesc> hd((size_t)n);
-    std::vector<uint8_t> st((size_t)n);
+    hd.resize((size_t)n); st.resize((size_t)n);
     CK(cudaMemcpyAsync(hd.data(), e->desc, (size_t)n * sizeof(ReadDesc), cudaMemcpyDeviceToHost, e->stream));
     CK(cudaMemcpyAsync(st.data(), e->state, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
     CK(cudaStreamSynchronize(e->stream));
-    bool changed = false;
-    for (int f = 0; f < e->n_files; ++f) {
-        std::priority_queue<int32_t, std::vector<int32_t>, std::greater<int32_t>> ends;  // accepted reads still buffered
-        bool have_prev = false; int32_t p_prev = 0;
-        for (int64_t i = e->h_file_start[f]; i < e->h_file_start[f + 1]; ++i) {
-            if (st[i] != ST_KEEP) continue;
-            const int32_t pos = hd[i].rpos, end = hd[i].rpos + e->h_rlen_tmp[i];
-            if (have_prev) {
-                while (!ends.empty() && ends.top() < p_prev) ends.pop();   // buffered = accepted reads with end >= previous accepted start
-                if (pos == p_prev && (int64_t)ends.size() + 1 > (int64_t)maxcnt) { st[i] = ST_MAXDROP; changed = true; continue; }
-            }
-            ends.push(end);
-            have_prev = true; p_prev = pos;
-        }
-    }
-    if (changed) CK(cudaMemcpyAsync(e->state, st.data(), (size_t)n, cudaMemcpyHostToDevice, e->stream));
-    e->maxdrop_applied = changed;
+    return 0;
+}
+
+// max-depth rule of bam_plp_push (apply_maxcnt), evaluated on the host only when a column could hold more than maxcnt reads
+static int apply_maxcnt_host(b200_engine *e, int64_t n, int maxcnt)
+{
+    std::vector<ReadDesc> hd; std::vector<uint8_t> st; std::vector<int32_t> rl((size_t)n);
+    CK(cudaMemcpyAsync(rl.data(), e->rlen, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
+    if (fetch_desc_state(e, n, hd, st)) return -1;
+    e->maxdrop_applied = apply_maxcnt(hd.data(), rl.data(), st.data(), e->h_file_start.data(), e->n_files, maxcnt);
+    if (e->maxdrop_applied) CK(cudaMemcpyAsync(e->state, st.data(), (size_t)n, cudaMemcpyHostToDevice, e->stream));
     return 0;
 }
 
@@ -745,32 +646,7 @@ __global__ void k_apply_maxdrop(const uint8_t *state, ReadDesc *desc, int32_t *e
 }
 
 static int stage_device(b200_engine *e, b200_stage_stats_t *stats);
-
-// Some record starts before its predecessor (rare path).  htslib's bam_plp_push rejects a PUSHED read that starts before
-// the previous pushed read of the same file ("The input is not sorted", error return); reads dropped by the filters never
-// reach the push.  The column kernels binary-search the descriptors by start, so unsorted input must not get through:
-// exact check over the kept reads of each file on the host.  depth (bam2depth.c:329-333) tolerates some disorder; here any
-// disorder among its kept reads is refused ("Data is not position sorted") rather than risking silently wrong counts.
-static int check_sorted_host(b200_engine *e, int64_t n)
-{
-    std::vector<ReadDesc> hd((size_t)n);
-    std::vector<uint8_t> st((size_t)n);
-    CK(cudaMemcpyAsync(hd.data(), e->desc, (size_t)n * sizeof(ReadDesc), cudaMemcpyDeviceToHost, e->stream));
-    CK(cudaMemcpyAsync(st.data(), e->state, (size_t)n, cudaMemcpyDeviceToHost, e->stream));
-    CK(cudaStreamSynchronize(e->stream));
-    for (int f = 0; f < e->n_files; ++f) {
-        bool have = false; int32_t last = 0;
-        for (int64_t i = e->h_file_start[f]; i < e->h_file_start[f + 1]; ++i) {
-            if (st[i] != ST_KEEP) continue;
-            if (have && hd[i].rpos < last) {
-                snprintf(e->err, sizeof e->err, "%s", e->sconf.mode == B200_MODE_DEPTH ? "Data is not position sorted" : "The input is not sorted (reads out of order)");
-                return -3;
-            }
-            have = true; last = hd[i].rpos;
-        }
-    }
-    return 0;
-}
+static TextDims text_dims(const b200_engine *e) { return {e->sum_rlen, e->sum_indel_text, e->ncols_max, e->name.size(), e->n_files, e->n}; }
 
 extern "C" int b200_stage(b200_engine_t *e, const b200_batch_t *b, const b200_stage_conf_t *cf, b200_stage_stats_t *stats)
 {
@@ -814,13 +690,7 @@ extern "C" int b200_stage(b200_engine_t *e, const b200_batch_t *b, const b200_st
     if (cf->mode == B200_MODE_DEPTH && cf->d_remove_overlaps && b->depth_clip && n > 0) {
         // clip coordinates replayed by the caller (one name hash per file, across reference sequences)
         e->h_clip_tmp.resize((size_t)n);
-        for (int64_t i = 0; i < n; ++i) {
-            const int64_t cabs = b->depth_clip[i];
-            int64_t rel = cabs ? cabs - e->win_base : (int64_t)INT32_MIN;
-            if (rel > INT32_MAX) rel = INT32_MAX;
-            if (rel < INT32_MIN) rel = INT32_MIN;
-            e->h_clip_tmp[(size_t)i] = (int32_t)rel;
-        }
+        for (int64_t i = 0; i < n; ++i) e->h_clip_tmp[(size_t)i] = clip_rel(b->depth_clip[i], e->win_base);
         H2D(clip, e->h_clip_tmp.data(), n);
         e->has_host_clip = true;
     }
@@ -877,21 +747,14 @@ static int stage_device(b200_engine *e, b200_stage_stats_t *stats)
     StageAcc ha;
     CK(cudaMemcpyAsync(&ha, e->d_acc, sizeof ha, cudaMemcpyDeviceToHost, e->stream));
     CK(cudaStreamSynchronize(e->stream));
-    if (ha.n_desc) { const int rc = check_sorted_host(e, n); if (rc) return rc; }
+    if (ha.n_desc) {   // rare path: some record starts before its predecessor
+        std::vector<ReadDesc> hd; std::vector<uint8_t> st;
+        if (fetch_desc_state(e, n, hd, st)) return -1;
+        if (const char *msg = check_sorted(hd.data(), st.data(), e->h_file_start.data(), e->n_files, cf->mode)) { snprintf(e->err, sizeof e->err, "%s", msg); return -3; }
+    }
     e->acc_n_kept = (int64_t)ha.n_kept; e->max_rend = ha.n_kept ? ha.max_rend : 0;
     e->sum_rlen = ha.sum_rlen; e->sum_indel_text = ha.sum_indel_text; e->sum_rlen_gen = ha.sum_rlen_gen;
-    // ---- column domain
-    {
-        int64_t wend = cf->end - e->win_base;                       // exclusive, relative
-        int64_t cov = e->max_rend > 0 ? e->max_rend : 0;
-        if (cov > wend) cov = wend;
-        int64_t allc = (cf->end < e->tid_len ? cf->end : e->tid_len) - e->win_base;
-        if (allc < 0) allc = 0;
-        e->ncols_cov = cov; e->ncols_all = allc;
-        int64_t nc = cov > allc ? cov : allc;
-        if (nc >= (1LL << 31) - 4096) { snprintf(e->err, sizeof e->err, "window too wide (%lld columns)", (long long)nc); return -1; }
-        e->ncols_max = (int32_t)nc;
-    }
+    if (!column_domain(e->max_rend, cf->end, e->tid_len, e->win_base, e->ncols_cov, e->ncols_all, e->ncols_max, e->err, sizeof e->err)) return -1;
     e->n_groups = (e->ncols_max + 31) / 32 + 1;
     ENSURE(glo, (size_t)e->n_groups * e->n_files + 1); ENSURE(ghi, (size_t)e->n_groups * e->n_files + 1);
     e->maxdrop_applied = false;
@@ -906,8 +769,6 @@ static int stage_device(b200_engine *e, b200_stage_stats_t *stats)
             may_fire = (int64_t)mb + 1 > (int64_t)cf->max_depth;
         }
         if (may_fire) {
-            e->h_rlen_tmp.resize((size_t)n);
-            CK(cudaMemcpyAsync(e->h_rlen_tmp.data(), e->rlen, (size_t)n * 4, cudaMemcpyDeviceToHost, e->stream));
             if (apply_maxcnt_host(e, n, cf->max_depth)) return -1;
             if (e->maxdrop_applied) {
                 k_apply_maxdrop<<<nblk(n, 256), 256, 0, e->stream>>>(e->state, e->desc, e->endv, n); e->launches++;
@@ -936,7 +797,7 @@ static int stage_device(b200_engine *e, b200_stage_stats_t *stats)
     if (stats) {
         stats->n_kept = (int64_t)ha.n_kept; stats->n_kept_in_window = (int64_t)ha.n_kept_in_window;
         stats->n_reads = ha.n_reads; stats->n_selected_reads = ha.n_selected; stats->summed_mapq = ha.summed_mapq;
-        stats->out_bound = e->text_bound(27, 1);
+        stats->out_bound = text_bound(text_dims(e), 27, 1);
         stats->n_cols = e->ncols_max;
     }
     return 0;
@@ -1030,33 +891,26 @@ static int upload_bed(b200_engine *e, const int64_t *bb, const int64_t *be, int 
     return 0;
 }
 
-template <class Fmt, class KS, class KW>
-static int run_text(b200_engine *e, KS k_size, KW k_write, const Fmt &fmt, uint64_t bound, char *out, size_t out_cap, size_t *out_len)
+// The text pass over nt 128-column tiles once the per-column buffers are in place: sizes() launches the size pass (line
+// lengths into col_n / col_state, tile totals into tile_total), a scan turns the tile totals into byte offsets (col_off),
+// write() launches the byte pass into e->out; then the timings, the bound check and the copy-out.
+template <class Sizes, class Write>
+static int text_pass(b200_engine *e, int nt, uint64_t bound, Sizes sizes, Write write, char *out, size_t out_cap, size_t *out_len)
 {
-    const int32_t ncols = fmt.v.ncols;
-    const int nt = (ncols + TILE - 1) / TILE;
-    *out_len = 0;
-    e->last_kernel_ms = 0;
-    if (nt == 0) return 0;
     ENSURE(out, (size_t)bound + 64);
-    unsigned long long total = 0;
-    typedef typename Fmt::State State;
-    ENSURE(col_n, (size_t)ncols + 1);                                   // per-column line length
-    const size_t st_words = ((size_t)ncols * sizeof(State) + 7) / 8 + 1;
-    ENSURE(col_state, st_words);                                        // per-column formatter state
     ENSURE(tile_total, (size_t)nt + 1); ENSURE(col_off, (size_t)nt + 2);
     const int nb = nblk(nt, 256);
     ENSURE(status, (size_t)nb + 1);
     CK(cudaMemsetAsync(e->status, 0, ((size_t)nb + 1) * 8, e->stream));
     CK(cudaMemsetAsync(e->d_misc, 0, 8, e->stream));
     CK(cudaEventRecord(e->ev0, e->stream));
-    k_size<<<nt, TILE, 0, e->stream>>>(fmt, e->col_n, (State *)e->col_state, e->tile_total); e->launches++;
+    if (sizes()) return -1;
     CK(cudaEventRecord(e->evA, e->stream));
     k_scan_u32_to_u64<<<nb, 256, 0, e->stream>>>(e->tile_total, e->col_off, nt, e->status, (uint32_t *)e->d_misc); e->launches++;
     CK(cudaEventRecord(e->evB, e->stream));
-    k_write<<<nt, TILE, e->smem_text + 16, e->stream>>>(fmt, e->col_n, (const State *)e->col_state, e->col_off, e->out, e->smem_text, e->use_tma);
-    e->launches++;
+    if (write()) return -1;
     CK(cudaEventRecord(e->ev1, e->stream));
+    unsigned long long total = 0;
     CK(cudaMemcpyAsync(&total, e->col_off + nt, 8, cudaMemcpyDeviceToHost, e->stream));
     CK(cudaStreamSynchronize(e->stream));
     CK(cudaGetLastError());
@@ -1064,7 +918,7 @@ static int run_text(b200_engine *e, KS k_size, KW k_write, const Fmt &fmt, uint6
     cudaEventElapsedTime(&ms, e->ev0, e->evA); e->last_parts_ms[0] = ms;      // size pass
     cudaEventElapsedTime(&ms, e->evA, e->evB); e->last_parts_ms[1] = ms;      // tile-offset scan
     cudaEventElapsedTime(&ms, e->evB, e->ev1); e->last_parts_ms[2] = ms;      // write pass
-    if (total > bound) { snprintf(e->err, sizeof e->err, "internal: output %llu exceeds bound %llu", total, (unsigned long long)bound); return -1; }
+    if (!within_bound(total, bound, e->err, sizeof e->err)) return -1;
     *out_len = (size_t)total;
     e->last_out_len = (size_t)total;
     if (out) {
@@ -1075,22 +929,26 @@ static int run_text(b200_engine *e, KS k_size, KW k_write, const Fmt &fmt, uint6
     return 0;
 }
 
-static uint64_t mpileup_bound(const b200_engine *e, const b200_mpileup_conf_t *c)
+// thread-per-column text: k_size / k_write over Fmt (text_size_tile / text_write_tile)
+template <class Fmt, class KS, class KW>
+static int run_text(b200_engine *e, KS k_size, KW k_write, const Fmt &fmt, uint64_t bound, char *out, size_t out_cap, size_t *out_len)
 {
-    const int per = 2 + (c->out_mapq ? 1 : 0) + (c->out_qpos ? 12 : 0) + (c->out_qpos5 ? 13 : 0);
-    uint64_t b = e->text_bound(per, 1 + 2 * (3 + c->n_star_cols));
-    if (c->n_x > 0 && c->x_off) {   // host columns: every (read, column) entry can add the read's strings + separators
-        uint64_t worst = 0;
-        for (int64_t i = 0; i < e->n; ++i) {
-            uint64_t w = 0;
-            for (int k = 0; k < c->n_x; ++k) { const uint32_t *o = c->x_off + (size_t)k * ((size_t)e->n + 1) + (size_t)i; w += (uint64_t)(o[1] - o[0]) + 1; }
-            worst = std::max(worst, w);
-        }
-        b += (uint64_t)e->sum_rlen * worst;
-    }
-    return b;
+    const int32_t ncols = fmt.v.ncols;
+    const int nt = (ncols + TILE - 1) / TILE;
+    *out_len = 0;
+    e->last_kernel_ms = 0;
+    if (nt == 0) return 0;
+    typedef typename Fmt::State State;
+    ENSURE(col_n, (size_t)ncols + 1);                                   // per-column line length
+    const size_t st_words = ((size_t)ncols * sizeof(State) + 7) / 8 + 1;
+    ENSURE(col_state, st_words);                                        // per-column formatter state
+    return text_pass(e, nt, bound,
+        [&] { k_size<<<nt, TILE, 0, e->stream>>>(fmt, e->col_n, (State *)e->col_state, e->tile_total); e->launches++; return 0; },
+        [&] { k_write<<<nt, TILE, e->smem_text + 16, e->stream>>>(fmt, e->col_n, (const State *)e->col_state, e->col_off, e->out, e->smem_text, e->use_tma); e->launches++; return 0; },
+        out, out_cap, out_len);
 }
-extern "C" uint64_t b200_mpileup_text_bound(const b200_engine_t *e, const b200_mpileup_conf_t *c) { return (e && e->staged && c) ? mpileup_bound(e, c) : 0; }
+
+extern "C" uint64_t b200_mpileup_text_bound(const b200_engine_t *e, const b200_mpileup_conf_t *c) { return (e && e->staged && c) ? mpileup_bound(text_dims(e), c) : 0; }
 
 extern "C" int b200_mpileup_text(b200_engine_t *e, const b200_mpileup_conf_t *c, char *out, size_t out_cap, size_t *out_len)
 {
@@ -1102,7 +960,7 @@ extern "C" int b200_mpileup_text(b200_engine_t *e, const b200_mpileup_conf_t *c,
     fmt.cf.min_baseQ = c->min_baseQ; fmt.cf.all = c->all; fmt.cf.rev_del = c->rev_del; fmt.cf.no_ins = c->no_ins;
     fmt.cf.no_del = c->no_del; fmt.cf.no_ends = c->no_ends; fmt.cf.out_mapq = c->out_mapq; fmt.cf.out_qpos = c->out_qpos;
     fmt.cf.out_qpos5 = c->out_qpos5; fmt.cf.n_star_cols = c->n_star_cols;
-    const uint64_t bound = mpileup_bound(e, c);
+    const uint64_t bound = mpileup_bound(text_dims(e), c);
     if (c->n_x > 0) {   // host columns: upload the per-read string tables, widen the bound by the longest per-read contribution
         if (c->n_x > PLP_MAX_X || c->n_x != c->n_star_cols || !c->x_off || (!c->x_dat && c->x_bytes)) { snprintf(e->err, sizeof e->err, "bad host-column tables"); return -1; }
         const size_t n_off = (size_t)c->n_x * ((size_t)e->n + 1);
@@ -1116,15 +974,9 @@ extern "C" int b200_mpileup_text(b200_engine_t *e, const b200_mpileup_conf_t *c,
     const int nt = (ncols + TILE - 1) / TILE;            // 128-column tiles
     *out_len = 0; e->last_kernel_ms = 0;
     if (nt == 0) return 0;
-    ENSURE(out, (size_t)bound + 64);
     ENSURE(col_n, (size_t)nt * TILE + 1);
     ENSURE(col_state, ((size_t)nt * TILE * sizeof(MpFileSz) + 7) / 8 + 1);
-    ENSURE(tile_total, (size_t)nt + 1); ENSURE(col_off, (size_t)nt + 2);
     ENSURE(ent, e->qual_bytes + 64 + ENT_PAD); ENSURE(ent2, (size_t)e->sum_rlen_gen + 64 + ENT_PAD);   // front pad + slack for the gather's 80-byte fetches
-    const int nb = nblk(nt, 256);
-    ENSURE(status, (size_t)nb + 1);
-    CK(cudaMemsetAsync(e->status, 0, ((size_t)nb + 1) * 8, e->stream));
-    CK(cudaMemsetAsync(e->d_misc, 0, 8, e->stream));
     ENSURE(ss_diff, (size_t)ncols + 2); ENSURE(ss_nplp, (size_t)ncols + 2); ENSURE(ss_fail, (size_t)ncols + 1); ENSURE(ss_extra, (size_t)ncols + 1);
     CK(cudaMemsetAsync(e->ss_diff, 0, ((size_t)ncols + 2) * 4, e->stream));
     CK(cudaMemsetAsync(e->ss_fail, 0, ((size_t)ncols + 1) * 4, e->stream));
@@ -1133,8 +985,8 @@ extern "C" int b200_mpileup_text(b200_engine_t *e, const b200_mpileup_conf_t *c,
     ENSURE(status2, (size_t)nbs + 1);
     CK(cudaMemsetAsync(e->status2, 0, ((size_t)nbs + 1) * 8, e->stream));
     CK(cudaMemsetAsync(e->d_misc + 2, 0, 16, e->stream));      // scan ticket, cursor of the second entry array
-    CK(cudaEventRecord(e->ev0, e->stream));
-    {
+    // entry strings + order-free line sizes
+    auto sizes = [&] {
         const int64_t want_blocks = (e->n * 32 + 255) / 256;
         const int rb = (int)std::max<int64_t>(1, std::min<int64_t>(want_blocks, (int64_t)e->n_sm * 16));
         if (e->has_ref) k_mp_entries<true><<<rb, 256, 0, e->stream>>>(fmt.v, fmt.cf, e->n, e->ref_codes, e->ss_diff, e->ss_fail, e->ss_extra, e->ent + ENT_PAD, e->ent2 + ENT_PAD, e->d_misc + 3, e->desc);
@@ -1142,11 +994,10 @@ extern "C" int b200_mpileup_text(b200_engine_t *e, const b200_mpileup_conf_t *c,
         e->launches++;
         k_ss_scan<<<nbs, 256, 0, e->stream>>>(e->ss_diff, e->ss_nplp, ncols + 1, e->status2, (uint32_t *)(e->d_misc + 2)); e->launches++;
         k_ss_cols<<<nt, TILE, 0, e->stream>>>(fmt.v, fmt.cf, e->ss_nplp, e->ss_fail, e->ss_extra, e->col_n, (MpFileSz *)e->col_state, e->tile_total); e->launches++;
-    }
-    CK(cudaEventRecord(e->evA, e->stream));
-    k_scan_u32_to_u64<<<nb, 256, 0, e->stream>>>(e->tile_total, e->col_off, nt, e->status, (uint32_t *)e->d_misc); e->launches++;
-    CK(cudaEventRecord(e->evB, e->stream));
-    {
+        return 0;
+    };
+    // gather
+    auto write = [&] {
         MpEntFmt gf; gf.v = fmt.v; gf.cf = fmt.cf; gf.E = e->ent + ENT_PAD; gf.E2 = e->ent2 + ENT_PAD;
         // the cold paths of the gather read the same structure from global memory (see mpileup_ent.cuh)
         if (!e->d_gfmt) CK(cudaMalloc(&e->d_gfmt, sizeof(MpEntFmt)));
@@ -1164,24 +1015,9 @@ extern "C" int b200_mpileup_text(b200_engine_t *e, const b200_mpileup_conf_t *c,
         if (c->out_mapq) k_mp_gather<7, true><<<nt, TILE, cap + 16, e->stream>>>(gf, dg, e->col_n, (const MpFileSz *)e->col_state, e->col_off, e->out, cap, e->use_tma);
         else k_mp_gather<7, false><<<nt, TILE, cap + 16, e->stream>>>(gf, dg, e->col_n, (const MpFileSz *)e->col_state, e->col_off, e->out, cap, e->use_tma);
         e->launches++;
-    }
-    CK(cudaEventRecord(e->ev1, e->stream));
-    unsigned long long total = 0;
-    CK(cudaMemcpyAsync(&total, e->col_off + nt, 8, cudaMemcpyDeviceToHost, e->stream));
-    CK(cudaStreamSynchronize(e->stream));
-    CK(cudaGetLastError());
-    float ms = 0; cudaEventElapsedTime(&ms, e->ev0, e->ev1); e->last_kernel_ms = ms;
-    cudaEventElapsedTime(&ms, e->ev0, e->evA); e->last_parts_ms[0] = ms;      // entry strings + sizes
-    cudaEventElapsedTime(&ms, e->evA, e->evB); e->last_parts_ms[1] = ms;      // tile-offset scan
-    cudaEventElapsedTime(&ms, e->evB, e->ev1); e->last_parts_ms[2] = ms;      // gather
-    if (total > bound) { snprintf(e->err, sizeof e->err, "internal: output %llu exceeds bound %llu", total, (unsigned long long)bound); return -1; }
-    *out_len = (size_t)total; e->last_out_len = (size_t)total;
-    if (out) {
-        if (total > out_cap) { snprintf(e->err, sizeof e->err, "output buffer too small: need %llu bytes", total); return -2; }
-        CK(cudaMemcpyAsync(out, e->out, (size_t)total, cudaMemcpyDeviceToHost, e->stream));
-        CK(cudaStreamSynchronize(e->stream));
-    }
-    return 0;
+        return 0;
+    };
+    return text_pass(e, nt, bound, sizes, write, out, out_cap, out_len);
 }
 
 extern "C" int b200_depth_text(b200_engine_t *e, const b200_depth_conf_t *c, char *out, size_t out_cap, size_t *out_len)
@@ -1192,15 +1028,9 @@ extern "C" int b200_depth_text(b200_engine_t *e, const b200_depth_conf_t *c, cha
     DpFmt fmt;
     fill_view(e, fmt.v, e->bed_beg, e->bed_end, c->n_bed, c->bed_active, c->all);
     fmt.cf.min_qual = c->min_qual; fmt.cf.count_del = c->count_del; fmt.cf.all = c->all;
-    const uint64_t ncols = (uint64_t)fmt.v.ncols;
-    const uint64_t bound = ncols * (e->name.size() + 1 + 20 + (uint64_t)e->n_files * 12 + 1) + 64;
-    return run_text(e, k_depth_size, k_depth_write, fmt, bound, out, out_cap, out_len);
+    return run_text(e, k_depth_size, k_depth_write, fmt, depth_bound((uint64_t)fmt.v.ncols, e->name.size(), e->n_files), out, out_cap, out_len);
 }
-extern "C" uint64_t b200_depth_text_bound(const b200_engine_t *e)
-{
-    if (!e || !e->staged) return 0;
-    return (uint64_t)e->ncols_max * (e->name.size() + 1 + 20 + (uint64_t)e->n_files * 12 + 1) + 64;
-}
+extern "C" uint64_t b200_depth_text_bound(const b200_engine_t *e) { return (e && e->staged) ? depth_bound((uint64_t)e->ncols_max, e->name.size(), e->n_files) : 0; }
 
 extern "C" int b200_coverage(b200_engine_t *e, const b200_coverage_conf_t *c, b200_coverage_sums_t *sums)
 {

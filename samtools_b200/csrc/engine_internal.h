@@ -60,13 +60,8 @@ struct b200_engine {
     size_t last_out_len = 0;
     uint64_t gl_rng_draws = 0;   // hts_drand48 draws consumed so far by errmod's ks_shuffle
     std::vector<int64_t> h_file_start;
-    std::vector<int32_t> h_rlen_tmp, h_clip_tmp;
+    std::vector<int32_t> h_clip_tmp;
 
-    uint64_t text_bound(int per_entry, int per_file_extra) const
-    {
-        return (uint64_t)sum_rlen * (uint64_t)per_entry + sum_indel_text +
-               (uint64_t)ncols_max * (name.size() + 24 + (uint64_t)n_files * (16 + (uint64_t)per_file_extra)) + 64;
-    }
     void free_all()
     {
         void *ps[] = { qual0, mapq0, pos, flag, mapq, l_qseq, n_cigar, cigar_off, qual_off, mtid, mpos, isize, prev, rbits, cigar, seq4, qual,

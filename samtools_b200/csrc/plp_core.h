@@ -149,6 +149,35 @@ PLP_HD ReadRange read_range(const View &v, int f, int g)
 }
 PLP_HD int32_t range_at(const ReadRange &r, int32_t t) { return t < r.n_ovf ? r.ovf[t] : r.lo + (t - r.n_ovf); }
 
+// The [first,last) slice of a file's reads [fs,fe) that can cover group g.  first is the later of (a) the first read whose
+// running max end (pmax, prefix max over the file) exceeds the group start and (b) the first read starting within kReach
+// columns of it; reads before (b) that still reach the group are listed separately (ovf_span), so one spliced read cannot
+// widen the slice of every group under it.
+PLP_HD void group_slice(const ReadDesc *desc, const int32_t *pmax, int64_t fs, int64_t fe, int32_t g, int64_t &first, int64_t &last)
+{
+    const int32_t c0 = g * 32, c1 = c0 + 31;
+    int64_t lo = fs, hi = fe;
+    while (lo < hi) { int64_t m = (lo + hi) >> 1; if (pmax[m] > c0) hi = m; else lo = m + 1; }   // first read whose running max end exceeds c0
+    first = lo;
+    lo = first; hi = fe;
+    while (lo < hi) { int64_t m = (lo + hi) >> 1; if (desc[m].rpos > c0 - kReach) hi = m; else lo = m + 1; }  // first read within reach
+    if (lo > first) first = lo;
+    lo = first; hi = fe;
+    while (lo < hi) { int64_t m = (lo + hi) >> 1; if (desc[m].rpos > c1) hi = m; else lo = m + 1; }  // first read starting beyond c1
+    last = lo > first ? lo : first;
+}
+
+// far-reaching reads: d is listed for the groups [g0,g1], those with 32g >= rpos + kReach and 32g < rend (false: none)
+PLP_HD bool ovf_span(const ReadDesc &d, int32_t n_groups, int32_t &g0, int32_t &g1)
+{
+    if ((int64_t)d.rend - d.rpos <= kReach) return false;
+    const int64_t a = (int64_t)d.rpos + kReach;
+    g0 = (int32_t)(a <= 0 ? 0 : (a + 31) >> 5);
+    g1 = d.rend > 0 ? (d.rend - 1) >> 5 : -1;
+    if (g1 >= n_groups) g1 = n_groups - 1;
+    return true;
+}
+
 struct MpConf {
     int32_t min_baseQ, all, rev_del, no_ins, no_del, no_ends, out_mapq, out_qpos, out_qpos5, n_star_cols;
 };
@@ -999,5 +1028,68 @@ PLP_HD void cv_column(const View &v, int32_t min_baseQ, int tile, int32_t c, CvC
         if (dpos > 0) { o.count_base = true; o.depth += (uint32_t)dpos; }
     }
 }
+
+// what a column adds to its bin of the histogram views (coverage.c:609-660): its depth, or 1 if covered (breadth)
+PLP_HD uint32_t cv_hist_add(const CvCol &o, int32_t min_depth, int plot_depth)
+{
+    return plot_depth ? o.depth : ((o.count_base && o.depth >= (uint32_t)min_depth) ? 1u : 0u);
+}
+
+// bedcov (bedcov.c:316-331): a column takes part when the multi-file iterator would return it (any file has a read over it)
+PLP_HD bool bc_any(const View &v, int32_t c)
+{
+    bool any = false;
+    for (int f = 0; f < v.n_files && !any; ++f) {
+        const ReadRange rr = read_range(v, f, c >> 5);
+        for (int32_t t_ = 0; t_ < rr.n && !any; ++t_) { const ReadDesc d = load_hot(v.desc + range_at(rr, t_)); any = (uint32_t)(c - d.rpos) < (uint32_t)(d.rend - d.rpos); }
+    }
+    return any;
+}
+// depth of file f at column c, without deletions / reference skips when skip_dn (simple reads have neither)
+PLP_HD int32_t bc_depth(const View &v, int f, int32_t c, int skip_dn)
+{
+    const ReadRange rr = read_range(v, f, c >> 5);
+    int32_t np = 0, m = 0;
+    for (int32_t t_ = 0; t_ < rr.n; ++t_) {
+        const int32_t i = range_at(rr, t_);
+        ReadDesc d = load_hot(v.desc + i);
+        if ((uint32_t)(c - d.rpos) >= (uint32_t)(d.rend - d.rpos)) continue;
+        ++np;
+        if (skip_dn && !(d.fl & RD_SIMPLE)) { load_cold(d, v.desc + i); Ent e; resolve(v, d, c, e); if (e.is_del || e.is_refskip) ++m; }
+    }
+    return np - m;
+}
+
+// depth rows "name\tpos(\tdepth)*\n" (bam2depth.c:234-244); size() keeps the first file's depth for write()
+struct DpFmt {
+    View v; DpConf cf;
+    struct State { int32_t d0; };
+    PLP_HD uint32_t size(int32_t c, State &s) const
+    {
+        bool any = false; uint32_t body = 0;
+        for (int f = 0; f < v.n_files; ++f) {
+            DpCol o; dp_file_column(v, cf, f, c >> 5, c, o);
+            if (f == 0) s.d0 = o.depth;
+            any |= o.spanned;
+            body += 1 + (uint32_t)ndigits((uint64_t)o.depth);
+        }
+        if (!any && !(cf.all && c < v.ncols_all)) return 0;
+        if (!bed_pass(v, c)) return 0;
+        return (uint32_t)v.name_len + 1 + (uint32_t)ndigits((uint64_t)(v.win_base + c + 1)) + body + 1;
+    }
+    PLP_HD void write(int32_t c, const State &s, char *p) const
+    {
+        for (int i = 0; i < v.name_len; ++i) *p++ = v.name[i];
+        *p++ = '\t';
+        p += put_u64(p, (uint64_t)(v.win_base + c + 1));
+        for (int f = 0; f < v.n_files; ++f) {
+            int32_t d = s.d0;
+            if (f) { DpCol o; dp_file_column(v, cf, f, c >> 5, c, o); d = o.depth; }
+            *p++ = '\t';
+            p += put_u64(p, (uint64_t)d);
+        }
+        *p = '\n';
+    }
+};
 
 }  // namespace plp

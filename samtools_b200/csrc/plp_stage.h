@@ -205,7 +205,7 @@ PLP_HD void stage_build_desc(const RawSoA &r, const b200_stage_conf_t &cf, int64
         }
     }
     desc[i] = d;
-    if (i > 0 && r.pos[i] < r.pos[i - 1]) PLP_ADD64(&acc->n_desc, 1);   // bam_plp_push rejects unsorted input; see check_sorted_host()
+    if (i > 0 && r.pos[i] < r.pos[i - 1]) PLP_ADD64(&acc->n_desc, 1);   // bam_plp_push rejects unsorted input; see check_sorted() in stage_host.h
     // end used for the running max that bounds the per-group read slices: capped at rpos + kReach, because from
     // there on the read is served through the far-reaching lists (k_ovf_*) and must not widen the slices under it
     endv[i] = d.rend > d.rpos ? (d.rend - d.rpos > kReach ? d.rpos + kReach : d.rend) : INT32_MIN;
@@ -434,5 +434,31 @@ PLP_HD void depth_clip_chain(const RawSoA &r, int64_t i, const int64_t *next, co
     }
 }
 
+// column-major pileup entries for the iterator tier: the number of file f's reads over column c, and, with Fill, their
+// entries in file order at o
+template <bool Fill>
+PLP_HD uint32_t column_entries(const View &v, int f, int32_t c, b200_pileup1_t *o)
+{
+    const ReadRange rr = read_range(v, f, c >> 5);
+    uint32_t n = 0;
+    for (int32_t t_ = 0; t_ < rr.n; ++t_) {
+        const int32_t i = range_at(rr, t_);
+        const ReadDesc d = v.desc[i];
+        if (c < d.rpos || c >= d.rend) continue;
+        ++n;
+        if (!Fill) continue;
+        Ent e; resolve(v, d, c, e);
+        if (e.k < 0) {   // simple read: the op index of its match
+            const uint32_t *cg = v.cigar + d.cig_off; int k = 0;
+            while (!is_mop(cg[k] & 0xf)) ++k;
+            e.k = k;
+        }
+        b200_pileup1_t p;
+        p.read = i; p.qpos = e.qpos; p.indel = e.indel; p.cigar_ind = e.k;
+        p.is_del = e.is_del; p.is_head = e.is_head; p.is_tail = e.is_tail; p.is_refskip = e.is_refskip;
+        *o++ = p;
+    }
+    return n;
+}
 
 }  // namespace plp

@@ -1,22 +1,19 @@
 // emul_engine.cpp -- DEBUG HARNESS, NOT PART OF THE PRODUCT.
 //
-// Implements the C ABI of include/b200_pileup.h by stepping the very same
-// __host__ __device__ per-read / per-column functions the CUDA kernels call
-// (samtools_b200/csrc/plp_core.h, plp_stage.h) in a plain single-threaded
-// loop.  It exists so that the column arithmetic and the host drivers can be
-// debugged in the dev container, which has no GPU.  It is built only by
-// tests/emul/build.sh, is never linked into libb200pileup.so or b200samtools,
-// is never used as a fallback, and is not a measured or shipped path.
+// Implements the C ABI of include/b200_pileup.h by stepping the very same __host__ __device__ per-read / per-column
+// functions the CUDA kernels call (samtools_b200/csrc/plp_core.h, plp_stage.h) and the engine's host-side policy
+// (stage_host.h).  Of its own it has only sequential loops in place of the kernel grids, a host prefix max in place of the
+// device scans, and the cross-checks below (reference implementations).  It exists so that the column arithmetic and the
+// host drivers can be debugged on a machine without a GPU.  It is built only by tests/emul/build.sh, is never linked into
+// libb200pileup.so or b200samtools, is never used as a fallback, and is not a measured or shipped path.
 // BAQ (warp-cooperative kernel) and GL are NOT emulated: calls needing them fail.
 #include "../../include/b200_pileup.h"
-#include "../../samtools_b200/csrc/plp_core.h"
-#include "../../samtools_b200/csrc/plp_stage.h"
+#include "../../samtools_b200/csrc/stage_host.h"
 #include <algorithm>
 #include <climits>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <queue>
 #include <string>
 #include <vector>
 
@@ -57,6 +54,7 @@ static RawSoA raw(b200_engine *e)
     return r;
 }
 
+// k_scan_max + k_ranges + k_ovf_*: a host prefix max in place of the device scan, then the same group_slice / ovf_span
 static void build_ranges(b200_engine *e, int *max_range)
 {
     const b200_batch_t &b = e->b;
@@ -70,29 +68,17 @@ static void build_ranges(b200_engine *e, int *max_range)
     *max_range = 0;
     for (int f = 0; f < b.n_files; ++f)
         for (int g = 0; g < e->n_groups; ++g) {
-            const int64_t fs = b.file_start[f], fe = b.file_start[f + 1];
-            const int32_t c0 = g * 32, c1 = c0 + 31;
-            int64_t lo = fs, hi = fe;
-            while (lo < hi) { int64_t m = (lo + hi) >> 1; if (e->pmax[(size_t)m] > c0) hi = m; else lo = m + 1; }
-            int64_t first = lo;
-            hi = fe;
-            while (lo < hi) { int64_t m = (lo + hi) >> 1; if (e->desc[(size_t)m].rpos > c0 - kReach) hi = m; else lo = m + 1; }
-            if (lo > first) first = lo;
-            lo = first; hi = fe;
-            while (lo < hi) { int64_t m = (lo + hi) >> 1; if (e->desc[(size_t)m].rpos > c1) hi = m; else lo = m + 1; }
-            const int64_t last = std::max(lo, first);
+            int64_t first, last;
+            group_slice(e->desc.data(), e->pmax.data(), b.file_start[f], b.file_start[f + 1], g, first, last);
             e->glo[(size_t)f * e->n_groups + g] = (int32_t)first; e->ghi[(size_t)f * e->n_groups + g] = (int32_t)last;
             *max_range = std::max(*max_range, (int)(last - first));
         }
-    // far-reaching reads per group (same rule as k_ovf_*)
+    // far-reaching reads per group, in file order
     std::vector<std::vector<int32_t>> lists((size_t)e->n_groups * b.n_files);
     for (int f = 0; f < b.n_files; ++f)
         for (int64_t i = b.file_start[f]; i < b.file_start[f + 1]; ++i) {
-            const ReadDesc &d = e->desc[(size_t)i];
-            if ((int64_t)d.rend - d.rpos <= kReach) continue;
-            const int64_t a = (int64_t)d.rpos + kReach;
-            int32_t g0 = (int32_t)(a <= 0 ? 0 : (a + 31) >> 5), g1 = d.rend > 0 ? (d.rend - 1) >> 5 : -1;
-            if (g1 >= e->n_groups) g1 = e->n_groups - 1;
+            int32_t g0, g1;
+            if (!ovf_span(e->desc[(size_t)i], e->n_groups, g0, g1)) continue;
             for (int32_t g = g0; g <= g1; ++g) lists[(size_t)f * e->n_groups + g].push_back((int32_t)i);
         }
     { size_t mo = 0; for (auto &l : lists) mo = std::max(mo, l.size()); *max_range += (int)mo; }
@@ -101,6 +87,8 @@ static void build_ranges(b200_engine *e, int *max_range)
     e->ovf_off[lists.size()] = (int32_t)e->ovf_idx.size(); e->ovf_off[lists.size() + 1] = (int32_t)e->ovf_idx.size();
     e->ovf_idx.push_back(0);
 }
+
+static TextDims text_dims(const b200_engine *e) { return {e->acc.sum_rlen, e->acc.sum_indel_text, e->ncols_max, e->name.size(), e->b.n_files, e->b.n_reads}; }
 
 int b200_stage(b200_engine_t *e, const b200_batch_t *b, const b200_stage_conf_t *cf, b200_stage_stats_t *stats)
 {
@@ -125,39 +113,17 @@ int b200_stage(b200_engine_t *e, const b200_batch_t *b, const b200_stage_conf_t 
     }
     for (int64_t i = 0; i < n; ++i) stage_prep2(r, *cf, i, e->state.data());
     for (int64_t i = 0; i < n; ++i) stage_build_desc(r, *cf, i, e->state.data(), e->rlen.data(), e->desc.data(), e->endv.data(), &e->acc, e->win_base, e->cig_x.data(), e->cig_y.data());
-    if (e->acc.n_desc)   // same rule as check_sorted_host() in engine.cu
-        for (int f = 0; f < b->n_files; ++f) {
-            bool have = false; int32_t last = 0;
-            for (int64_t i = b->file_start[f]; i < b->file_start[f + 1]; ++i) {
-                if (e->state[(size_t)i] != ST_KEEP) continue;
-                if (have && e->desc[(size_t)i].rpos < last) { e->err = cf->mode == B200_MODE_DEPTH ? "Data is not position sorted" : "The input is not sorted (reads out of order)"; return -3; }
-                have = true; last = e->desc[(size_t)i].rpos;
-            }
-        }
-    const int32_t max_rend = e->acc.n_kept ? e->acc.max_rend : 0;
-    int64_t wend = cf->end - e->win_base, cov = max_rend > 0 ? max_rend : 0;
-    if (cov > wend) cov = wend;
-    int64_t allc = std::min<int64_t>(cf->end, b->tid_len) - e->win_base; if (allc < 0) allc = 0;
-    e->ncols_cov = cov; e->ncols_all = allc; e->ncols_max = (int32_t)std::max(cov, allc);
+    if (e->acc.n_desc)
+        if (const char *msg = check_sorted(e->desc.data(), e->state.data(), b->file_start, b->n_files, cf->mode)) { e->err = msg; return -3; }
+    char msg[128];
+    if (!column_domain(e->acc.n_kept ? e->acc.max_rend : 0, cf->end, b->tid_len, e->win_base, e->ncols_cov, e->ncols_all, e->ncols_max, msg, sizeof msg)) {
+        e->err = msg; return -1;
+    }
     e->n_groups = (e->ncols_max + 31) / 32 + 1;
     int max_range = 0;
     build_ranges(e, &max_range);
     if (cf->mode != B200_MODE_DEPTH && cf->max_depth > 0 && 2LL * max_range + 1 > (int64_t)cf->max_depth) {
-        bool changed = false;
-        for (int f = 0; f < b->n_files; ++f) {
-            std::priority_queue<int32_t, std::vector<int32_t>, std::greater<int32_t>> ends;
-            bool have = false; int32_t pp = 0;
-            for (int64_t i = b->file_start[f]; i < b->file_start[f + 1]; ++i) {
-                if (e->state[(size_t)i] != ST_KEEP) continue;
-                const int32_t pos = e->desc[(size_t)i].rpos, end = pos + e->rlen[(size_t)i];
-                if (have) {
-                    while (!ends.empty() && ends.top() < pp) ends.pop();
-                    if (pos == pp && (int64_t)ends.size() + 1 > (int64_t)cf->max_depth) { e->state[(size_t)i] = ST_MAXDROP; changed = true; continue; }
-                }
-                ends.push(end); have = true; pp = pos;
-            }
-        }
-        if (changed) {
+        if (apply_maxcnt(e->desc.data(), e->rlen.data(), e->state.data(), b->file_start, b->n_files, cf->max_depth)) {
             for (int64_t i = 0; i < n; ++i) if (e->state[(size_t)i] == ST_MAXDROP) { e->desc[(size_t)i].rend = e->desc[(size_t)i].rpos; e->endv[(size_t)i] = INT32_MIN; }
             build_ranges(e, &max_range);
         }
@@ -165,12 +131,7 @@ int b200_stage(b200_engine_t *e, const b200_batch_t *b, const b200_stage_conf_t 
     e->has_clip = false;
     if (cf->mode == B200_MODE_DEPTH && cf->d_remove_overlaps && b->depth_clip) {
         e->clip.assign((size_t)n + 1, INT32_MIN);
-        for (int64_t i = 0; i < n; ++i) {
-            int64_t rel = b->depth_clip[i] ? b->depth_clip[i] - e->win_base : (int64_t)INT32_MIN;
-            if (rel > INT32_MAX) rel = INT32_MAX;
-            if (rel < INT32_MIN) rel = INT32_MIN;
-            e->clip[(size_t)i] = (int32_t)rel;
-        }
+        for (int64_t i = 0; i < n; ++i) e->clip[(size_t)i] = clip_rel(b->depth_clip[i], e->win_base);
         e->has_clip = true;
     } else if (b->prev_same_name && ((cf->mode == B200_MODE_MPILEUP && cf->overlaps) || (cf->mode == B200_MODE_DEPTH && cf->d_remove_overlaps))) {
         e->next.assign((size_t)n + 1, -1);
@@ -190,7 +151,7 @@ int b200_stage(b200_engine_t *e, const b200_batch_t *b, const b200_stage_conf_t 
         memset(stats, 0, sizeof *stats);
         stats->n_kept = (int64_t)e->acc.n_kept; stats->n_kept_in_window = (int64_t)e->acc.n_kept_in_window;
         stats->n_reads = e->acc.n_reads; stats->n_selected_reads = e->acc.n_selected; stats->summed_mapq = e->acc.summed_mapq;
-        stats->out_bound = 0; stats->n_cols = e->ncols_max;
+        stats->out_bound = text_bound(text_dims(e), 27, 1); stats->n_cols = e->ncols_max;
     }
     return 0;
 }
@@ -211,8 +172,11 @@ static void fill_view(b200_engine *e, View &v, const int64_t *bb, const int64_t 
     v.n_x = 0; v.x_stride = 0; v.x_off = nullptr; v.x_dat = nullptr; memset(v.x_sep, 0, sizeof v.x_sep);
 }
 
-static int emit(b200_engine *e, const std::string &s, char *out, size_t cap, size_t *out_len)
+// the tail of the engine's text pass: bound check, then the copy-out
+static int emit(b200_engine *e, const std::string &s, uint64_t bound, char *out, size_t cap, size_t *out_len)
 {
+    char msg[128];
+    if (!within_bound(s.size(), bound, msg, sizeof msg)) { e->err = msg; return -1; }
     *out_len = s.size();
     if (out) { if (s.size() > cap) { e->err = "output buffer too small"; return -2; } memcpy(out, s.data(), s.size()); }
     return 0;
@@ -312,35 +276,24 @@ int b200_mpileup_text(b200_engine_t *e, const b200_mpileup_conf_t *c, char *out,
         if (use_ent) mp_line_write_ent(v, cf, col, s0, &s[at], E.data(), E2.data());
         else mp_line_write(v, cf, col >> 5, col, s0, &s[at]);
     }
-    return emit(e, s, out, cap, out_len);
+    return emit(e, s, mpileup_bound(text_dims(e), c), out, cap, out_len);
 }
 
-uint64_t b200_mpileup_text_bound(const b200_engine_t *e, const b200_mpileup_conf_t *c)
-{
-    size_t n = 0;
-    return b200_mpileup_text(const_cast<b200_engine_t *>(e), c, nullptr, 0, &n) == 0 ? n + 64 : 0;
-}
-int b200_depth_text(b200_engine_t *e, const b200_depth_conf_t *c, char *out, size_t cap, size_t *out_len);
-uint64_t b200_depth_text_bound(const b200_engine_t *e)
-{
-    // every row: name, tab, position, (tab, depth) per file, newline
-    return (uint64_t)e->ncols_max * (e->name.size() + 1 + 20 + (uint64_t)e->b.n_files * 12 + 1) + 64;
-}
+uint64_t b200_mpileup_text_bound(const b200_engine_t *e, const b200_mpileup_conf_t *c) { return e->staged && c ? mpileup_bound(text_dims(e), c) : 0; }
+uint64_t b200_depth_text_bound(const b200_engine_t *e) { return e->staged ? depth_bound((uint64_t)e->ncols_max, e->name.size(), e->b.n_files) : 0; }
 int b200_depth_text(b200_engine_t *e, const b200_depth_conf_t *c, char *out, size_t cap, size_t *out_len)
 {
-    View v; fill_view(e, v, c->bed_beg, c->bed_end, c->n_bed, c->bed_active, c->all);
-    DpConf cf{c->min_qual, c->count_del, c->all};
+    DpFmt fmt; fill_view(e, fmt.v, c->bed_beg, c->bed_end, c->n_bed, c->bed_active, c->all);
+    fmt.cf = DpConf{c->min_qual, c->count_del, c->all};
     std::string s;
-    for (int32_t col = 0; col < v.ncols; ++col) {
-        bool any = false; std::vector<int32_t> d((size_t)v.n_files);
-        for (int f = 0; f < v.n_files; ++f) { DpCol o; dp_file_column(v, cf, f, col >> 5, col, o); d[(size_t)f] = o.depth; any |= o.spanned; }
-        if (!any && !(cf.all && col < v.ncols_all)) continue;
-        if (!bed_pass(v, col)) continue;
-        s += e->name; s += '\t'; s += std::to_string(v.win_base + col + 1);
-        for (int f = 0; f < v.n_files; ++f) { s += '\t'; s += std::to_string(d[(size_t)f]); }
-        s += '\n';
+    for (int32_t col = 0; col < fmt.v.ncols; ++col) {
+        DpFmt::State st{};
+        const uint32_t len = fmt.size(col, st);
+        if (!len) continue;
+        const size_t at = s.size(); s.resize(at + len, '?');
+        fmt.write(col, st, &s[at]);
     }
-    return emit(e, s, out, cap, out_len);
+    return emit(e, s, depth_bound((uint64_t)fmt.v.ncols, e->name.size(), fmt.v.n_files), out, cap, out_len);
 }
 
 int b200_coverage(b200_engine_t *e, const b200_coverage_conf_t *c, b200_coverage_sums_t *sums)
@@ -359,7 +312,7 @@ int b200_coverage_hist(b200_engine_t *e, const b200_coverage_conf_t *c, int64_t 
     View v; fill_view(e, v, nullptr, nullptr, 0, 0, 0);
     for (int32_t col = 0; col < v.ncols; ++col) {
         CvCol o; cv_column(v, c->min_baseQ, col >> 5, col, o);
-        const uint32_t add = plot_depth ? o.depth : ((o.count_base && o.depth >= (uint32_t)c->min_depth) ? 1u : 0u);
+        const uint32_t add = cv_hist_add(o, c->min_depth, plot_depth);
         const int64_t bin = ((int64_t)col - (beg - v.win_base)) / bin_width;
         if (add && bin >= 0 && bin < n_bins) hist[bin] += add;
     }
@@ -368,29 +321,22 @@ int b200_coverage_hist(b200_engine_t *e, const b200_coverage_conf_t *c, int64_t 
 int b200_bedcov(b200_engine_t *e, int32_t skip_dn, int32_t min_depth, uint64_t *cnt, uint64_t *pcov)
 {
     View v; fill_view(e, v, nullptr, nullptr, 0, 0, 0);
-    const bool dn = skip_dn || min_depth >= 0;
+    const int dn = skip_dn || min_depth >= 0;
     for (int f = 0; f < v.n_files; ++f) { cnt[f] = 0; if (pcov) pcov[f] = 0; }
     for (int32_t c = 0; c < v.ncols; ++c) {
-        std::vector<int32_t> pd((size_t)v.n_files, 0); bool any = false;
+        if (!bc_any(v, c)) continue;
         for (int f = 0; f < v.n_files; ++f) {
-            const ReadRange rr = read_range(v, f, c >> 5);
-            for (int32_t t_ = 0; t_ < rr.n; ++t_) {
-                const int32_t i = range_at(rr, t_);
-                const ReadDesc d = v.desc[i];
-                if (c < d.rpos || c >= d.rend) continue;
-                any = true; ++pd[(size_t)f];
-                if (dn) { Ent en; resolve(v, d, c, en); if (en.is_del || en.is_refskip) --pd[(size_t)f]; }
-            }
+            const int32_t d = bc_depth(v, f, c, dn);
+            cnt[f] += (uint64_t)d;
+            if (pcov && min_depth >= 0 && d >= min_depth) pcov[f]++;
         }
-        if (!any) continue;
-        for (int f = 0; f < v.n_files; ++f) { cnt[f] += (uint64_t)pd[(size_t)f]; if (pcov && min_depth >= 0 && pd[(size_t)f] >= min_depth) pcov[f]++; }
     }
     return 0;
 }
 int b200_glf(b200_engine_t *e, int32_t, int64_t *, int64_t *, int32_t *, float *, float *, size_t) { e->err = "emulation harness: GL not emulated"; return -1; }
 int b200_fetch_qual(b200_engine_t *e, uint8_t *q, size_t cap) { memcpy(q, e->qual.data(), std::min(cap, e->qual.size())); return 0; }
 int b200_fetch_mapq_keep(b200_engine_t *e, uint8_t *m, uint8_t *k, size_t n) { n = std::min(n, (size_t)e->b.n_reads); if (m) memcpy(m, e->mapq.data(), n); if (k) memcpy(k, e->state.data(), n); return 0; }
-// column-major (read, column) entries: the same per-column walk as k_entries_count / k_entries_fill (engine.cu)
+// column-major (read, column) entries: column_entries per column, counts first (k_entries_count / k_entries_fill in engine.cu)
 int b200_pileup_entries(b200_engine_t *e, int32_t file, int64_t beg, int64_t end, uint32_t *col_n, b200_pileup1_t *ents, size_t cap, size_t *n_out)
 {
     if (!e->staged) { e->err = "no staged batch"; return -1; }
@@ -401,27 +347,11 @@ int b200_pileup_entries(b200_engine_t *e, int32_t file, int64_t beg, int64_t end
     if (re > v.ncols) re = v.ncols;
     *n_out = 0;
     if (re <= rb) return 0;
-    std::vector<b200_pileup1_t> all;
-    for (int64_t c64 = rb; c64 < re; ++c64) {
-        const int32_t c = (int32_t)c64;
-        const ReadRange rr = read_range(v, file, c >> 5);
-        uint32_t n = 0;
-        for (int32_t t_ = 0; t_ < rr.n; ++t_) {
-            const int32_t i = range_at(rr, t_);
-            const ReadDesc d = v.desc[i];
-            if (c < d.rpos || c >= d.rend) continue;
-            Ent en; resolve(v, d, c, en);
-            if (en.k < 0) { const uint32_t *cg = v.cigar + d.cig_off; int k = 0; while (!is_mop(cg[k] & 0xf)) ++k; en.k = k; }
-            b200_pileup1_t p; memset(&p, 0, sizeof p);
-            p.read = i; p.qpos = en.qpos; p.indel = en.indel; p.cigar_ind = en.k;
-            p.is_del = en.is_del; p.is_head = en.is_head; p.is_tail = en.is_tail; p.is_refskip = en.is_refskip;
-            all.push_back(p); ++n;
-        }
-        col_n[c64 - rb] = n;
-    }
-    *n_out = all.size();
-    if (all.size() > cap) { e->err = "entry buffer too small"; return -2; }
-    if (!all.empty()) memcpy(ents, all.data(), all.size() * sizeof(b200_pileup1_t));
+    size_t ne = 0;
+    for (int64_t c = rb; c < re; ++c) { col_n[c - rb] = column_entries<false>(v, file, (int32_t)c, nullptr); ne += col_n[c - rb]; }
+    *n_out = ne;
+    if (ne > cap) { e->err = "entry buffer too small"; return -2; }
+    for (int64_t c = rb; c < re; ++c) ents += column_entries<true>(v, file, (int32_t)c, ents);
     return 0;
 }
 }

@@ -1,11 +1,15 @@
 """Host drivers + per-column / per-read arithmetic, single-stepped on the CPU.
 
 tests/emul/emul_engine.cpp implements the C ABI by calling the very same
-__host__ __device__ functions the CUDA kernels call (plp_core.h, plp_stage.h),
-so the b200samtools driver code (option handling, -a/-aa sequencing, packing,
-BED / RG / BQ-tag host bits) and the column formatter can be checked against
-the reference's golden outputs without a GPU.  This harness is a debugging aid,
-not a product path: it is never linked into libb200pileup.so / b200samtools.
+__host__ __device__ functions the CUDA kernels call (plp_core.h, plp_stage.h)
+and the engine's host-side policy (stage_host.h: max-depth sweep, sortedness,
+column domain, text bounds).  What it does on its own is only the control flow:
+sequential loops in place of the kernel grids and a host prefix max in place of
+the device scans.  So the b200samtools driver code (option handling, -a/-aa
+sequencing, packing, BED / RG / BQ-tag host bits), the column formatters and
+the output bounds can be checked against the reference's golden outputs without
+a GPU.  This harness is a debugging aid, not a product path: it is never linked
+into libb200pileup.so / b200samtools.
 The BAQ kernel (warp-cooperative) is not emulated: those cases run in -m gpu."""
 import os, subprocess
 import pytest
